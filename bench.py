@@ -2,7 +2,7 @@
 """Headline benchmark: user-item pairs scored / second (fused top-k) at rank 50.
 
     python bench.py --gpus N --steps K --warmup W            (our arm)
-    python bench.py --impl reference --gpus N --steps K ...  (the reference's own CPU path, baseline/_ref)
+    python bench.py --impl reference --gpus N --steps K ...  (the reference's own CPU path, oracle/_ref)
 
 Workload (BASELINE.json configs[1], "C2"): synthetic 1M users x 100K items, ~0.1% nnz (1e8 interactions, Zipf item
 popularity, log-normal user degrees), SVDModel rank 50, filter_seen, top-10, every user scored against every item.
@@ -20,6 +20,11 @@ What the JSON line carries besides the contract keys:
   e2e_csr_fastpath      same call fed with a ready-made pinned host CSR (3x fewer bytes over PCIe)
   build_e2e_s           build() from host triplets: H2D + ingest + transpose + panels + randomized SVD
   cpu_baseline          the reference (polara) itself on this box's host cores: default knobs and tuned knobs
+
+--dump-outputs DIR writes what the last timed step returned to DIR/<name>.npy (see dump_outputs): the top-k lists for
+c2, the factors and core of the CoFFee build for c4, the lists of every rank of the sweep for c5.  The inputs are seeded
+and identical from run to run, so two builds can be compared output for output.  bench.py runs on the library build()
+made, refuses one that is missing or older than its sources, and writes nothing into the tree (no compile, no bytecode).
 
 Multi-GPU (weak scaling in items, SURVEY.md 8e): every rank owns a 100K-item shard of the item factors (total items =
 N x 100K); user embeddings are computed row-sharded (each rank its block of users) and all-gathered; per-shard top-k
@@ -42,6 +47,8 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True
+DUMP_BYTES = 64 << 20
 
 
 def parse_args():
@@ -67,7 +74,47 @@ def parse_args():
                     help="c2 (default; with --users/--items/--nnz/--rank/--gpus also C3's shape), c4 = CoFFee HOOI on a "
                          "1M x 50K x 5 tensor, c5 = ScaledSVD rank sweep on 5M x 500K (one build at rank 500)")
     ap.add_argument("--scale", type=float, default=1.0, help="c4/c5: shrink users, items and nnz by this factor")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
+
+
+def require_built_library():
+    """The numbers must be those of the current sources: a library that is missing or older than them is an error
+    (build() makes it; bench.py compiles nothing, so that it can run from a read-only tree)."""
+    from polara_b200 import _build
+    if _build.needs_build():
+        raise SystemExit("%s is missing or older than its sources: run build() first" % _build.LIB_PATH)
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every ``name -> array`` to ``out_dir/<name>.npy``: floating arrays in float64 when they are float64, else
+    float32; integer arrays (item ids) in float32 when below 2**24, else float64 -- exact either way.  At most DUMP_BYTES
+    in all: the budget is shared out smallest array first, and an array larger than its share is replaced by a fixed,
+    seeded sample of its rows, whose row numbers go to ``<name>_rows.npy`` (float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BYTES - 2 * 128 * len(arrays)          # .npy headers: 128 bytes for each of at most two files an array
+    names = sorted(arrays, key=lambda k: arrays[k].size)
+    for n, name in enumerate(names):
+        a = np.asarray(arrays[name])
+        if a.dtype == np.float64 or (a.dtype.kind in "iu" and a.size and np.abs(a).max() >= 2 ** 24):
+            a = a.astype(np.float64)
+        else:
+            a = a.astype(np.float32)
+        share = left // (len(names) - n)
+        if a.nbytes > share:
+            row_bytes = a[0].nbytes + 8
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], share // row_bytes, replace=False))
+            a = a[rows]
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+            left -= rows.size * 8
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        left -= a.nbytes
 
 
 # ------------------------------------------------------------------ data ------------
@@ -152,7 +199,7 @@ def load_peaks():
 
 # ------------------------------------------------------------- CPU baseline ---------
 def reference_baseline(triplets, shape, v64, topk, budget_s):
-    """The reference itself (polara, from baseline/_ref) on this box's host cores: SVDModel.get_recommendations()'s own
+    """The reference itself (polara, from oracle/_ref) on this box's host cores: SVDModel.get_recommendations()'s own
     chunk driver over the first chunks of users with the FULL test arrays in place (so each chunk pays what it pays in
     the full job, models.py:260-270), (i) library defaults (memory_hard_limit 1 GiB, no thread pool,
     polara/recommender/defaults.py:50-51) and (ii) tuned (larger chunks + max_test_workers), as BASELINE.md 2 promises.
@@ -255,11 +302,10 @@ def run_c4(args):
     (the reference cannot run r2 = 5 on 5 levels: ARPACK needs k < min(shape), lib/tensor.py:78-79).  One step = one HOOI
     iteration (three TTMs + three thin SVDs).  Roofline: the mode-0 TTM against its algorithmic bytes (SURVEY.md 8d)."""
     import torch
-    from polara_b200 import _build
-    _build.build()
     from polara_b200.engine import get_engine
     from polara_b200.host import ArrayData
     from polara_b200.models import B200CoffeeModel
+    require_built_library()
     torch.cuda.set_device(0)
     dev = torch.device("cuda", 0)
     eng = get_engine(0)
@@ -275,11 +321,13 @@ def run_c4(args):
     model.mlrank = (60, 60, 4)
     model.seed = 0
     model.growth_tol = 0.0                         # run exactly num_iters iterations
-    iters_w, iters_t = max(1, min(args.warmup, 2)), max(2, args.steps)
+    iters_w, iters_t = max(1, min(args.warmup, 2)), args.steps
     model.num_iters = iters_w
     model.build(); torch.cuda.synchronize()
     model.num_iters = iters_w + iters_t
     t0 = time.perf_counter(); model.build(); torch.cuda.synchronize(); t_all = time.perf_counter() - t0
+    if args.dump_outputs:          # the build whose last iteration is the last timed step
+        dump_outputs(args.dump_outputs, {k: model.factors[k] for k in ("userid", "itemid", "rating", "core")})
     model.num_iters = iters_w
     t0 = time.perf_counter(); model.build(); torch.cuda.synchronize(); t_w = time.perf_counter() - t0
     s_per_iter = (t_all - t_w) / iters_t
@@ -310,12 +358,11 @@ def run_c5(args):
     pipelines.py:81-116).  Every rank runs the tcgen05 kernel (K-slab pipeline above rank 61)."""
     import torch
     import warnings
-    from polara_b200 import _build
-    _build.build()
     from polara_b200.engine import DeviceCSR, get_engine
     from polara_b200.host import ArrayData
     from polara_b200.models import B200ScaledSVD
     from polara_b200 import dist as pdist
+    require_built_library()
     torch.cuda.set_device(0)
     dev = torch.device("cuda", 0)
     eng = get_engine(0)
@@ -338,14 +385,22 @@ def run_c5(args):
     peaks = load_peaks(); peak_tf = float(peaks.get("bf16_tflops", 1590.0))
     pairs = float(n_users) * float(n_items)
     sweep = []
+    lists = {}
     for rank in (500, 200, 100, 50, 10):
         model.rank = rank
         v_dev = model._device_factor("itemid")
         step = pdist.make_step(eng, p_dev, v_dev, rank, args.topk, None)
         step(); torch.cuda.synchronize()
         s0 = eng.stats()
-        ms = timed(step, max(1, min(args.steps, 3)), torch.cuda.synchronize)
+        last = [None]
+
+        def run_step():
+            last[0] = step()
+        ms = timed(run_step, args.steps, torch.cuda.synchronize)
         s1 = eng.stats()
+        if args.dump_outputs:       # copied now: the next steps may reuse the engine's result buffers
+            lists["ids_rank%d" % rank] = last[0].cpu().numpy()
+        del last
         eng.set_prune(False)
         ms_full = timed(step, 1, torch.cuda.synchronize)
         fused_full = eng.last_score_kernel_ms()
@@ -355,6 +410,8 @@ def run_c5(args):
                       "executed_share": (s1[5] - s0[5]) / max(s1[6] - s0[6], 1),
                       "on_tensor_cores": (s1[6] - s0[6]) > 0})
         del step, v_dev
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, lists)
     best50 = [x for x in sweep if x["rank"] == 50][0]
     out = {"metric": "user-item pairs scored/sec (fused top-k) at rank 50", "value": best50["value"], "unit": "pairs/s", "n_gpus": 1,
            "steps": args.steps, "warmup": 1, "ms_per_step": best50["ms_per_step"], "higher_is_better": True, "scaling": "weak",
@@ -401,8 +458,7 @@ def main():
     dev = torch.device("cuda", local_rank)
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
-    from polara_b200 import _build
-    _build.build()
+    require_built_library()
     from polara_b200.engine import DeviceCSR, get_engine
     from polara_b200.host import ArrayData
     from polara_b200.models import B200SVDModel
@@ -485,6 +541,11 @@ def main():
         barrier()
     stop.set(); th.join()
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs:
+        # copied now: later variant steps may reuse the engine's result buffers
+        last = ids.cpu().numpy() if world == 1 else pdist.gather_lists(ids.cpu().numpy(), sharder, args.users, dev)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"ids": last})
     stats1 = eng.stats()
     launches = stats1[0] - stats0[0]
     if world > 1:
@@ -681,7 +742,7 @@ def main():
 
 
 def run_reference(args, base, n_items_total):
-    """Reference arm: the UNMODIFIED reference (polara, installed into baseline/_ref) scores a bounded sample of the
+    """Reference arm: the UNMODIFIED reference (polara, installed into oracle/_ref by build()) scores a bounded sample of the
     workload per step through its own chunk driver on the host cores; no GPU, none of our code on the path (the data
     generator is numpy; the data stub replays test_to_coo)."""
     from oracle import ref_driver as rd
@@ -741,7 +802,7 @@ def run_reference(args, base, n_items_total):
     out = dict(base)
     out.update({"impl": "reference", "value": value, "ms_per_step": dt * 1e3, "dtype": "f64",
                 "cpu_baseline": {"value": value, "unit": "pairs/s", "cores": cores, "kind": "reference",
-                                 "sample": "polara SVDModel chunk driver (baseline/_ref, unmodified), %s knobs: %d users "
+                                 "sample": "polara SVDModel chunk driver (oracle/_ref, unmodified), %s knobs: %d users "
                                            "(%d chunks of %d) x %d items per step, full-size test arrays in place"
                                            % (which, per_step_users, cfg["chunks_per_step"], cfg["chunk_users"], n_items_total),
                                  "settings": settings, "host": host},

@@ -1,9 +1,10 @@
 """Drive the UNMODIFIED reference (evfro/polara) on plain arrays  --  TEST INFRASTRUCTURE.
 
 Used by ``bench.py --impl reference`` / the ``cpu_baseline`` leg (timing the reference's
-own CPU path on the GPU box's host cores) and by the drop-in tests.  The reference is
-imported from ``baseline/_ref`` (the offline ``pip install --target`` of ``/root/reference``,
-git-ignored, travels to the GPU box) or, in the build container, from ``/root/reference``.
+own CPU path on the host cores) and by the drop-in tests.  The reference is imported
+from ``oracle/_ref`` (the git-ignored install ``build()`` makes with oracle/install_ref.py,
+so it goes wherever the tree is copied) or else from the checkout ``oracle.ref_shim``
+names.
 Nothing of ``polara_b200`` (models, kernels, engine) is on this path.
 
 The reference's models read their inputs from a ``RecommenderData`` object
@@ -21,9 +22,10 @@ from collections import namedtuple
 
 import numpy as np
 
-_HERE = os.path.dirname(os.path.abspath(__file__))
-_REF_CANDIDATES = (os.path.join(os.path.dirname(_HERE), "baseline", "_ref"),
-                   os.environ.get("POLARA_REFERENCE_ROOT", "/root/reference"))
+from oracle.install_ref import TARGET as _INSTALLED
+from oracle.ref_shim import REFERENCE_ROOT as _CHECKOUT
+
+_REF_CANDIDATES = (_INSTALLED, _CHECKOUT)
 
 Fields = namedtuple("Fields", "userid itemid feedback")
 _Index = namedtuple("Index", "userid itemid feedback")

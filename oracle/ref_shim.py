@@ -1,10 +1,13 @@
-"""Import the real reference (``/root/reference``) in the BUILD CONTAINER only.
+"""Import the real reference from a polara checkout.
 
-TEST INFRASTRUCTURE.  Used by ``oracle/make_golden.py`` (fixture generation) and
-by ``tests/test_oracle_vs_reference.py`` (skipped when the checkout is absent,
-e.g. on the GPU box).  The reference is untouched; pandas>=3 removed two private
-attributes it reads (``GroupBy.grouper`` at recommender/data.py:487,704-708 and
-``BaseGrouper.group_info``), which we re-expose here before importing it.
+TEST INFRASTRUCTURE.  ``REFERENCE_ROOT`` is the checkout: the directory named by
+the ``POLARA_REFERENCE_ROOT`` environment variable, or the default below when the
+variable is unset.  Used by ``oracle/make_golden.py`` (fixture generation), and
+as the source ``oracle/install_ref.py`` copies into ``oracle/_ref``; the pandas
+shim is also applied by ``oracle/ref_driver.py``.  The reference is untouched;
+pandas>=3 removed two private attributes it reads (``GroupBy.grouper`` at
+recommender/data.py:487,704-708 and ``BaseGrouper.group_info``), which we
+re-expose here before importing it.
 """
 import os
 import sys

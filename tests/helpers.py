@@ -36,6 +36,36 @@ def check_topk_against_scores(ids, scores64, seen_rows, seen_cols, k, tol):
     return exact / (m * k)
 
 
+def ratings_digest(user, item, fdbk):
+    """sha256 of seeded ratings (int64 user and item ids, float64 feedback): a fixture that stores a split instead of
+    the ratings records it, so that a change of the generator shows as changed inputs, not as a disagreement."""
+    import hashlib
+    h = hashlib.sha256()
+    for a, dtype in ((user, np.int64), (item, np.int64), (fdbk, np.float64)):
+        h.update(np.ascontiguousarray(a, dtype=dtype).tobytes())
+    return h.hexdigest()
+
+
+def replay_split(user, item, fdbk, g):
+    """What the reference's ``RecommenderData.prepare()`` hands a model for the ratings ``(user, item, fdbk)``, rebuilt
+    from the split it recorded in the fixture ``g`` (oracle/make_golden.py ``_record_split``): ``(train, test)``, each a
+    ``(user, item, fdbk)`` triplet in the data model's new indices and in the original row order.  Training keeps the
+    rows of the training users, test keeps the test users' rows that are not held out and whose item is in training.
+    Feedback values are passed through unchanged."""
+    def index_of(old, size):
+        new = np.full(size, -1, dtype=np.int64)
+        new[old] = np.arange(len(old))
+        return new
+    tr_user = index_of(g["train_user_old"], user.max() + 1)[user]
+    ts_user = index_of(g["test_user_old"], user.max() + 1)[user]
+    new_item = index_of(g["item_old"], item.max() + 1)[item]
+    train = tr_user >= 0
+    test = (ts_user >= 0) & (new_item >= 0)
+    test[g["holdout_rows"]] = False
+    return ((tr_user[train], new_item[train], fdbk[train]),
+            (ts_user[test], new_item[test], fdbk[test]))
+
+
 def random_seen_csr(rng, m, n, per_row):
     rows, cols = [], []
     for u in range(m):

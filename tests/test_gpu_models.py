@@ -280,12 +280,12 @@ def test_scaled_svd_rank_sweep_at_scale():
 
 def test_dropin_classes_against_the_real_reference():
     """polara_b200.models.dropin(): our device mixins grafted on the REAL polara classes, driven by a real RecommenderData
-    (needs the reference: baseline/_ref travels to the GPU box).  Same data object for both: singular values, subspace,
+    (needs the reference: build() installs it into oracle/_ref, which travels with the tree).  Same data object for both: singular values, subspace,
     lists and evaluate() hit counts vs polara's own SVDModel."""
     pd = pytest.importorskip("pandas")
     from oracle import ref_driver as rd
     if rd.reference_root() is None:
-        pytest.skip("reference not installed (baseline/_ref)")
+        pytest.skip("reference not installed (oracle/_ref)")
     rd.import_reference()
     from polara.recommender.data import RecommenderData
     from polara.recommender.models import SVDModel

@@ -1,79 +1,62 @@
-"""Oracle vs the LIVE reference on fresh seeds (build container only; skipped
-where /root/reference does not exist, e.g. on the GPU box)."""
+"""Oracle vs the reference, on what the reference computed from seeded inputs (``tests/golden/ref_*.npz``, recorded by
+``oracle/make_golden.py``).  CPU only; the reference itself is not needed to run them."""
 import numpy as np
 import pytest
 import scipy.sparse as sps
 
 from oracle import polara_oracle as po
-from oracle.ref_shim import import_reference, reference_available
+from polara_b200.synth import planted_ratings
+from tests.helpers import ratings_digest, replay_split
 
-pytestmark = pytest.mark.skipif(not reference_available(), reason="reference checkout absent")
+
+def _planted_split(g):
+    n_users, n_items, per_user, rank, seed = (int(x) for x in g["planted"])
+    ratings = planted_ratings(n_users, n_items, per_user, rank=rank, seed=seed)
+    assert ratings_digest(*ratings) == str(g["planted_sha256"]), \
+        "fixture inputs changed: planted_ratings no longer reproduces the ratings the reference was run on"
+    return replay_split(*ratings, g)
 
 
 @pytest.mark.parametrize("seed", [1, 2])
-def test_downvote_topk_rescale_live(seed):
-    import_reference()
-    from polara.recommender.models import RecommenderModel
-    from polara.preprocessing.matrices import rescale_matrix
-    rng = np.random.default_rng(seed)
-    s = rng.standard_normal((20, 50))
-    rows = np.repeat(np.arange(20), 4)
-    cols = np.concatenate([rng.choice(50, 4, replace=False) for _ in range(20)])
+def test_downvote_topk_rescale_live(golden, seed):
+    g = golden("ref_downvote_topk_rescale_s%d" % seed)
+    s = g["scores"]
     ref = s.copy()
-    RecommenderModel.downvote_seen_items(ref, (rows, cols))
-    mine = po.downvote_seen_items(s.copy(), rows, cols)
+    ref[g["seen_rows"], g["seen_cols"]] = g["downvoted_seen"]         # the rest of the block is left as it was
+    mine = po.downvote_seen_items(s.copy(), g["seen_rows"], g["seen_cols"])
     np.testing.assert_array_equal(mine, ref)
     for row in range(20):
-        np.testing.assert_array_equal(po.topsort(ref[row], 6), RecommenderModel.topsort(ref[row], 6))
-    a = sps.random(40, 30, density=0.2, random_state=seed, format="csr")
-    for scaling, axis in ((0.4, 0), (0.8, 1), (1, 0)):
-        np.testing.assert_allclose(po.rescale_matrix(a, scaling, axis).toarray(),
-                                   rescale_matrix(a, scaling, axis).toarray(), rtol=1e-14)
+        np.testing.assert_array_equal(po.topsort(ref[row], 6), g["topsort6"][row])
+    a = sps.csr_matrix((g["a_data"], g["a_indices"], g["a_indptr"]), shape=tuple(g["a_shape"]))
+    for (scaling, axis), rescaled in zip(g["rescale_cases"], g["rescaled"]):
+        np.testing.assert_allclose(po.rescale_matrix(a, scaling, int(axis)).toarray(), rescaled, rtol=1e-14)
 
 
-def test_hooi_live():
-    import_reference()
-    from polara.lib.tensor import hooi
-    rng = np.random.default_rng(3)
-    shp = (40, 30, 5)
-    nnz = 900
-    idx = np.unique(np.stack([rng.integers(0, s, nnz) for s in shp], axis=1), axis=0).astype(np.intp)
-    val = np.ones(len(idx))
-    ref = hooi(idx, val, shp, (4, 3, 2), num_iters=6, growth_tol=1e-4, seed=5)
-    mine = po.hooi(idx, val, shp, (4, 3, 2), num_iters=6, growth_tol=1e-4, seed=5)
-    for a, b in zip(mine[:3], ref[:3]):
+def test_hooi_live(golden):
+    g = golden("ref_hooi")
+    mine = po.hooi(g["idx"].astype(np.intp), g["val"], tuple(g["shape"]), tuple(g["mlrank"]),
+                   num_iters=int(g["num_iters"]), growth_tol=float(g["growth_tol"]), seed=int(g["seed"]))
+    for a, b in zip(mine[:3], (g["u0"], g["u1"], g["u2"])):
         sv = np.linalg.svd(a.T @ b, compute_uv=False)
         assert sv.min() > 1 - 1e-9
-    np.testing.assert_allclose(np.linalg.norm(mine[3]), np.linalg.norm(ref[3]), rtol=1e-10)
+    np.testing.assert_allclose(np.linalg.norm(mine[3]), np.linalg.norm(g["core"]), rtol=1e-10)
 
 
-def test_c1_shaped_svd_model_live():
-    """BASELINE config C1 (ML-1M shape: 6040 x 3706, ~1.0e6 ratings, PureSVD rank 10, top-10) through the REAL reference
+def test_c1_shaped_svd_model_live(golden):
+    """BASELINE config C1 (ML-1M shape: 6040 x 3706, ~1.0e6 ratings, PureSVD rank 10, top-10) as the reference ran it
     (RecommenderData.prepare + SVDModel.build + get_recommendations with its default chunking) against the oracle on the
-    arrays the reference's data model hands over: singular values, item-factor subspace, and every recommendation list
+    arrays the reference's data model handed over: singular values, item-factor subspace, and every recommendation list
     (scored with the reference's own factors: exact; with the oracle's factors: up to near-ties)."""
-    import pandas as pd
-    import_reference()
-    from polara.recommender.data import RecommenderData
-    from polara.recommender.models import SVDModel
-    from polara_b200.synth import planted_ratings
-    u, i, r = planted_ratings(6040, 3706, 166, rank=12, seed=11)
-    assert len(u) == 6040 * 166
-    data = RecommenderData(pd.DataFrame({"userid": u, "itemid": i, "rating": r}), "userid", "itemid", "rating", seed=0)
-    data.verbose = False
-    data.prepare()
-    model = SVDModel(data)
-    model.verbose = False
-    model.rank = 10
-    model.build()
-    recs = model.get_recommendations()
-    idx, val, shp = data.to_coo(tensor_mode=False)
-    a = sps.csr_matrix((val, (idx[:, 0], idx[:, 1])), shape=shp, dtype=np.float64)
-    v, s, _ = po.svd_build(a, 10)
-    np.testing.assert_allclose(s, model.factors["singular_values"], rtol=1e-9)
-    vref = model.factors[data.fields.itemid]
+    g = golden("ref_c1_svd")
+    (u, i, r), (tu, ti, tf) = _planted_split(g)
+    assert len(g["test_user_old"]) == 1208 and len(u) + len(tf) + len(g["holdout_rows"]) == 6040 * 166
+    a = sps.csr_matrix((r, (u, i)), shape=tuple(g["train_shape"]), dtype=np.float64)
+    v, s, _ = po.svd_build(a, int(g["rank"]))
+    np.testing.assert_allclose(s, g["singular_values"], rtol=1e-9)
+    vref = g["item_factors"].astype(np.float64)
     assert np.linalg.svd(v.T @ vref, compute_uv=False).min() > 1 - 1e-6
-    (tu, ti, tf), tshape, _ = model._get_test_data()
+    recs = g["recs"]
+    tshape = tuple(g["test_shape"])
     mine = po.recommend_svd(tu, ti, tf, tshape, vref, topk=10)
     assert mine.shape == recs.shape and recs.shape[1] == 10
     np.testing.assert_array_equal(mine, recs)
@@ -81,72 +64,46 @@ def test_c1_shaped_svd_model_live():
     assert (own == recs).mean() > 0.99
 
 
-def test_coffee_model_live_default_mlrank():
-    """CoffeeModel with the reference's default multilinear rank (13, 10, 2) on a 1500 x 600 x 5 tensor through the REAL
-    reference against the oracle: HOOI from the same seed (factor subspaces, core norm) and every recommendation list
+def test_coffee_model_live_default_mlrank(golden):
+    """CoffeeModel with the reference's default multilinear rank (13, 10, 2) on a 1500 x 600 x 5 tensor as the reference
+    ran it, against the oracle: HOOI from the same seed (factor subspaces, core norm) and every recommendation list
     scored with the reference's factors."""
-    import pandas as pd
-    import_reference()
-    from polara.recommender.data import RecommenderData
-    from polara.recommender.models import CoffeeModel
-    from polara_b200.synth import planted_ratings
-    u, i, r = planted_ratings(1500, 600, 40, rank=6, seed=13)
-    data = RecommenderData(pd.DataFrame({"userid": u, "itemid": i, "rating": r}), "userid", "itemid", "rating", seed=0)
-    data.verbose = False
-    data.prepare()
-    model = CoffeeModel(data)
-    model.verbose = False
-    model.seed = 3
-    model.num_iters = 8
-    model.build()
-    recs = model.get_recommendations()
-    idx, val, shp = data.to_coo(tensor_mode=True)
-    mine = po.hooi(idx.astype(np.intp), val, shp, tuple(model.mlrank), num_iters=model.num_iters,
-                   growth_tol=model.growth_tol, seed=model.seed)
-    f = data.fields
-    for got, key in zip(mine[:3], (f.userid, f.itemid, f.feedback)):
-        assert np.linalg.svd(got.T @ model.factors[key], compute_uv=False).min() > 1 - 1e-6, key
-    np.testing.assert_allclose(np.linalg.norm(mine[3]), np.linalg.norm(model.factors["core"]), rtol=1e-8)
-    (tu, ti, tf), tshape, _ = model._get_test_data()
-    lists = po.recommend_coffee(tu, ti, np.asarray(tf, dtype=np.int64), tshape, model.factors[f.itemid],
-                                model.factors[f.feedback], topk=10)
-    np.testing.assert_array_equal(lists, recs)
+    g = golden("ref_coffee_default_mlrank")
+    assert tuple(g["mlrank"]) == (13, 10, 2)
+    (u, i, r), (tu, ti, tf) = _planted_split(g)
+    level = lambda f: np.searchsorted(g["fdbk_old"], f)       # noqa: E731  (tensor mode: feedback -> level index)
+    idx = np.stack([u, i, level(r)], axis=1).astype(np.intp)
+    mine = po.hooi(idx, np.ones(len(idx)), tuple(g["train_shape"]), tuple(g["mlrank"]), num_iters=int(g["num_iters"]),
+                   growth_tol=float(g["growth_tol"]), seed=int(g["seed"]))
+    for got, key in zip(mine[:3], ("u0", "u1", "u2")):
+        assert np.linalg.svd(got.T @ g[key].astype(np.float64), compute_uv=False).min() > 1 - 1e-6, key
+    np.testing.assert_allclose(np.linalg.norm(mine[3]), np.linalg.norm(g["core"]), rtol=1e-8)
+    lists = po.recommend_coffee(tu, ti, level(tf).astype(np.int64), tuple(g["test_shape"]),
+                                g["u1"].astype(np.float64), g["u2"].astype(np.float64), topk=10)
+    np.testing.assert_array_equal(lists, g["recs"])
 
 
-def test_round_core_live():
+def test_round_core_live(golden):
     """CoffeeModel.round_core / _check_reduced_rank (models.py:949-980) against the oracle restatement."""
-    import_reference()
-    from polara.recommender.models import CoffeeModel
-    rng = np.random.default_rng(9)
-    core = rng.standard_normal((7, 6, 4))
-    for mode, rank in ((0, 3), (1, 6), (1, 2), (2, 1), (2, 3)):
-        rot_ref, core_ref = CoffeeModel.round_core(core, mode, rank)
+    g = golden("ref_round_core")
+    core = g["core"]
+    for c, (mode, rank) in enumerate(g["cases"]):
+        mode, rank = int(mode), int(rank)
         rot, new_core = po.round_core(core, mode, rank)
-        np.testing.assert_allclose(rot, rot_ref, rtol=0, atol=1e-13)
-        np.testing.assert_allclose(new_core, core_ref, rtol=0, atol=1e-13)
+        np.testing.assert_allclose(rot, g["rot%d" % c], rtol=0, atol=1e-13)
+        np.testing.assert_allclose(new_core, g["core%d" % c], rtol=0, atol=1e-13)
         assert new_core.shape[mode] == rank
 
 
 @pytest.mark.parametrize("switch_positive", [None, 4])
-def test_simple_rates_match_reference_live(switch_positive):
+def test_simple_rates_match_reference_live(golden, switch_positive):
     """evaluate(simple_rates=True) / holdout_size == 1 (models.py:451-458): hit rate, ARHR and MRR of the host mirror
     against the reference's own evaluation functions on random lists."""
-    import pandas as pd
-    import_reference()
-    from polara.recommender.evaluation import assemble_scoring_matrices, get_hr_score, get_rr_scores
     from polara_b200.host import evaluate_lists
-    rng = np.random.default_rng(12)
-    m, n, k = 60, 90, 10
-    recs = np.stack([rng.choice(n, k, replace=False) for _ in range(m)])
-    hu = np.repeat(np.arange(m), 3)
-    hi = np.concatenate([rng.choice(n, 3, replace=False) for _ in range(m)])
-    hf = rng.integers(1, 6, size=len(hu)).astype(np.float64)
-    holdout = pd.DataFrame({"userid": hu, "itemid": hi, "rating": hf})
-    is_positive = None if switch_positive is None else (hf >= switch_positive)
-    data = assemble_scoring_matrices(recs, holdout, "userid", "itemid", is_positive, feedback="rating")
-    hr_ref, rr_ref = get_hr_score(data[1]), get_rr_scores(data[1])
-    rel, rank = evaluate_lists(recs, hu, hi, hf, n, metric_type=["relevance", "ranking"], switch_positive=switch_positive,
-                               simple_rates=True)
-    np.testing.assert_allclose(rel.hr, hr_ref.hr, rtol=1e-12)
-    np.testing.assert_allclose(rank.arhr, rr_ref.arhr, rtol=1e-12)
-    np.testing.assert_allclose(rank.mrr, rr_ref.mrr, rtol=1e-12)
+    g = golden("ref_simple_rates")
+    tag = "none" if switch_positive is None else str(switch_positive)
+    rel, rank = evaluate_lists(g["recs"], g["holdout_user"], g["holdout_item"], g["holdout_fdbk"], int(g["n_items"]),
+                               metric_type=["relevance", "ranking"], switch_positive=switch_positive, simple_rates=True)
+    np.testing.assert_allclose(rel.hr, g["hr_" + tag], rtol=1e-12)
+    np.testing.assert_allclose(rank.arhr, g["arhr_" + tag], rtol=1e-12)
+    np.testing.assert_allclose(rank.mrr, g["mrr_" + tag], rtol=1e-12)
