@@ -292,6 +292,29 @@ int pb200_coo_group(pb200_ctx* ctx, int64_t nnz, int64_t n_keys, const int32_t* 
                     const int32_t* a, const int32_t* b, const float* val,
                     int64_t* seg_ptr, int32_t* a_out, int32_t* b_out, float* val_out);
 
+/* ProbabilisticMF build (models.py:743-770 -> generalized_sgd_sweep, polara/lib/optimize.py:123-250), stratified:
+ * users and items are cut into `strata` = B contiguous ranges (row_bounds / col_bounds, device int64 [B + 1], ascending,
+ * first 0, last n_rows / n_cols; empty ranges allowed).  Sub-epoch s processes the blocks (b, (b + s) mod B),
+ * b = 0..B-1, which share no user and no item; an epoch is the reference's sweep over the interactions permuted into
+ * (s, b) block order, reference (row-major) order inside a block.  B = 1 is the reference's own order.
+ * pb200_sgd_plan (once per build): from the training CSR (sorted, duplicates summed; zeros dropped by the caller) and
+ * the indptr of its transpose, writes block_ptr int64 [B*B + 1] (block s*B + b starts at block_ptr[s*B + b]), the
+ * permuted triplets users_out / items_out int32 [nnz], vals_out float32 [nnz], and the row / column nnz counts
+ * row_cnt_out int32 [n_rows], col_cnt_out int32 [n_cols] (getnnz(axis=1/0)).  1 <= B <= min(n_rows, n_cols, 65535). */
+int pb200_sgd_plan(pb200_ctx* ctx, int64_t n_rows, int64_t n_cols, int64_t nnz, const int64_t* indptr,
+                   const int32_t* indices, const float* values, const int64_t* t_indptr, int strata,
+                   const int64_t* row_bounds, const int64_t* col_bounds, int64_t* block_ptr,
+                   int32_t* users_out, int32_t* items_out, float* vals_out, int32_t* row_cnt_out, int32_t* col_cnt_out);
+
+/* One epoch of the plan's sweep, in place on the fp64 factors P [n_rows x ldp] and Q [n_cols x ldq] (row-major, rank
+ * <= 512 columns used): err = a - P[m].Q[n]; P[m] += learn_rate * (err Q[n] - P[m] lambd / row_cnt[m]);
+ * Q[n] += learn_rate * (err P[m] - Q[n] lambd / col_cnt[n]), both gradients from the old rows, fp64 without FMA
+ * contraction.  *cum_error_host (HOST) = sum of err^2 (per block in processing order, then over blocks in (s, b)
+ * order).  Deterministic: no atomics.  Synchronises the stream. */
+int pb200_sgd_epoch(pb200_ctx* ctx, int strata, const int64_t* block_ptr, const int32_t* users, const int32_t* items,
+                    const float* vals, const int32_t* row_cnt, const int32_t* col_cnt, double* P, int64_t ldp,
+                    double* Q, int64_t ldq, int rank, double learn_rate, double lambd, double* cum_error_host);
+
 #ifdef __cplusplus
 }
 #endif

@@ -66,6 +66,9 @@ _SIGNATURES = {
     "pb200_ttm_reduce": ([ptr, C.c_int, i64, ptr, ptr, ptr, ptr, ptr, C.c_int, i64, ptr, C.c_int, i64, ptr, i64],
                          C.c_int),
     "pb200_coo_group": ([ptr, i64, i64, ptr, ptr, ptr, ptr, ptr, ptr, ptr, ptr], C.c_int),
+    "pb200_sgd_plan": ([ptr, i64, i64, i64, ptr, ptr, ptr, ptr, C.c_int, ptr, ptr, ptr, ptr, ptr, ptr, ptr, ptr], C.c_int),
+    "pb200_sgd_epoch": ([ptr, C.c_int, ptr, ptr, ptr, ptr, ptr, ptr, ptr, i64, ptr, i64, C.c_int, f64, f64,
+                         C.POINTER(f64)], C.c_int),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

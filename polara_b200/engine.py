@@ -58,6 +58,36 @@ class DeviceCSR:
         return self.indptr.numel() * 8 + self.indices.numel() * 4 + self.values.numel() * 4
 
 
+def sgd_strata_bounds(counts, strata):
+    """Cut rows (or columns) with nnz ``counts`` into ``strata`` contiguous ranges with balanced nnz: range b < B-1
+    ends after the first row whose cumulative nnz reaches ceil((b+1) * nnz / B), the last range ends at the last row
+    (DESIGN.md 3.6).  Ranges may be empty (one row holding more than nnz / B).  Returns the B + 1 bounds (int64)."""
+    counts = np.asarray(counts, dtype=np.int64)
+    total = int(counts.sum())
+    if total <= 0:
+        raise ValueError("sgd_strata_bounds: no interactions")
+    targets = -(-np.arange(1, strata, dtype=np.int64) * total // strata)          # ceil((b+1) nnz / B), b < B-1
+    ends = np.searchsorted(np.cumsum(counts), targets, side="left") + 1
+    return np.concatenate(([0], ends, [len(counts)])).astype(np.int64)
+
+
+class SgdPlan:
+    """Device buffers of a stratified SGD schedule (pb200_sgd_plan): the training interactions permuted into processing
+    order (``users`` / ``items`` int32, ``vals`` float32), ``block_ptr`` [B*B + 1] (block s*B + b of sub-epoch s),
+    the row / column nnz counts, and the host-side range bounds of the cut."""
+
+    __slots__ = ("strata", "shape", "nnz", "row_bounds", "col_bounds", "block_ptr", "users", "items", "vals",
+                 "row_cnt", "col_cnt")
+
+    def __init__(self, **kw):
+        for k, v in kw.items():
+            setattr(self, k, v)
+
+    def permutation(self):
+        """the processing order as (user, item, value) host arrays."""
+        return self.users.cpu().numpy(), self.items.cpu().numpy(), self.vals.cpu().numpy()
+
+
 class _StreamFollowingLib:
     """Every C-ABI call runs on torch's CURRENT stream of the engine's device: tensors are allocated, uploaded and waited
     for relative to that stream (``torch.cuda.current_stream``), so the library context must enqueue on the same one.  When
@@ -450,6 +480,42 @@ class Engine:
                                        a.stride(0), _p(b, _F32), rb, b.stride(0), _p(out), ra * rb)
         self._check(st, "ttm_reduce")
         return out
+
+    def sgd_plan(self, a: DeviceCSR, strata):
+        """stratified schedule of the training CSR ``a`` (sorted, duplicates summed, no zero values) with ``strata``
+        user and item ranges (pb200_sgd_plan); the cut is made on the host from the row / column counts."""
+        if a.n_panels != 1:
+            raise ValueError("sgd_plan: needs a plain CSR")
+        n_rows, n_cols = a.shape
+        strata = int(strata)
+        at = self.transpose(a)
+        row_bounds = sgd_strata_bounds(np.diff(a.indptr.cpu().numpy()), strata)
+        col_bounds = sgd_strata_bounds(np.diff(at.indptr.cpu().numpy()), strata)
+        plan = SgdPlan(strata=strata, shape=(n_rows, n_cols), nnz=a.nnz, row_bounds=row_bounds, col_bounds=col_bounds,
+                       block_ptr=self.empty((strata * strata + 1,), _I64), users=self.empty((a.nnz,), _I32),
+                       items=self.empty((a.nnz,), _I32), vals=self.empty((a.nnz,), _F32),
+                       row_cnt=self.empty((n_rows,), _I32), col_cnt=self.empty((n_cols,), _I32))
+        rb, cb = self.upload(row_bounds), self.upload(col_bounds)
+        st = self.lib.pb200_sgd_plan(self.h, n_rows, n_cols, a.nnz, _p(a.indptr, _I64), _p(a.indices, _I32),
+                                     _p(a.values, _F32), _p(at.indptr, _I64), strata, _p(rb, _I64), _p(cb, _I64),
+                                     _p(plan.block_ptr), _p(plan.users), _p(plan.items), _p(plan.vals), _p(plan.row_cnt),
+                                     _p(plan.col_cnt))
+        self._check(st, "sgd_plan")
+        self.sync()                               # the bound arrays and the transpose are released on return
+        return plan
+
+    def sgd_epoch(self, plan: SgdPlan, p, q, rank, learn_rate, lam):
+        """one stratified SGD epoch in place on the float64 factors ``p`` [n_users x ld] / ``q`` [n_items x ld];
+        returns the epoch's sum of squared errors (pb200_sgd_epoch)."""
+        if p.shape[0] != plan.shape[0] or q.shape[0] != plan.shape[1]:
+            raise ValueError("sgd_epoch: factor shapes do not match the plan")
+        cum = C.c_double(0.0)
+        st = self.lib.pb200_sgd_epoch(self.h, plan.strata, _p(plan.block_ptr, _I64), _p(plan.users, _I32),
+                                      _p(plan.items, _I32), _p(plan.vals, _F32), _p(plan.row_cnt, _I32),
+                                      _p(plan.col_cnt, _I32), _p(p, _F64), p.stride(0), _p(q, _F64), q.stride(0),
+                                      int(rank), float(learn_rate), float(lam), C.byref(cum))
+        self._check(st, "sgd_epoch")
+        return float(cum.value)
 
 
 _ENGINES = {}

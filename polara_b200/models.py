@@ -22,7 +22,8 @@ import torch
 from . import host
 from .engine import DeviceCSR, get_engine, round_up
 
-__all__ = ["B200SVDModel", "B200ScaledSVD", "B200CoffeeModel", "dropin", "default_ell"]
+__all__ = ["B200SVDModel", "B200ScaledSVD", "B200CoffeeModel", "B200ProbabilisticMF", "dropin", "dropin_pmf",
+           "default_ell", "DEFAULT_SGD_STRATA"]
 
 
 def default_ell(rank, oversample=None):
@@ -907,6 +908,165 @@ class B200CoffeeModel(_CoffeeDeviceMixin, host.RecommenderModel):
 
     def build(self):
         return _CoffeeDeviceMixin.build(self)
+
+
+# ------------------------------------------------------------- ProbabilisticMF ------
+DEFAULT_SGD_STRATA = 1024     # user / item ranges of the stratified SGD epoch (DESIGN.md 3.6: chosen at C2 on a B200)
+
+
+def _padded_f32(arr, width_multiple=32):
+    r = arr.shape[1]
+    buf = np.zeros((arr.shape[0], round_up(r, width_multiple)), dtype=np.float32)
+    buf[:, :r] = arr
+    return buf
+
+
+class _PMFDeviceMixin(_DeviceModelMixin):
+    """Device implementation of ProbabilisticMF.build / get_recommendations (polara/recommender/models.py:728-787).
+    ``build()`` runs the reference's SGD sweep (lib/optimize.py:123-250) in fp64 on the device, in a stratified order
+    whose ``sgd_strata`` user and item ranges let disjoint blocks run concurrently (pb200_sgd_epoch, DESIGN.md 3.6);
+    ``sgd_strata = 1`` is the reference's own order.  Scoring is the fused kernel on ``P[test_users]`` and ``Q``."""
+
+    sgd_strata = DEFAULT_SGD_STRATA   # changes the result like ``seed`` does: part of the algorithm, not a speed switch
+
+    def _check_device_pmf(self, args, kwargs):
+        if args or kwargs:
+            raise NotImplementedError("ProbabilisticMF.build arguments %s (gradient adjusters such as adjust_gradient) "
+                                      "are not on the device path" % (list(args) + sorted(kwargs),))
+        opt = getattr(self, "optimizer", None)
+        if opt is not None and (getattr(opt, "__name__", None), getattr(opt, "__module__", None)) != \
+                ("simple_pmf_sgd", "polara.lib.optimize"):
+            raise NotImplementedError("optimizer %r is not on the device path: only simple_pmf_sgd is" % (opt,))
+        shard = getattr(self, "shard", None)
+        if shard is not None and shard.world > 1:
+            raise NotImplementedError("ProbabilisticMF on an item-sharded model")
+
+    def _pmf_training_csr(self):
+        """training triplets of ``to_coo`` -> device CSR (duplicates summed, zero values dropped: the reference's
+        ``.nonzero()`` drops them from the indices only, INTEGRATION.md)."""
+        idx, val, shape = self.data.to_coo(tensor_mode=False, feedback_threshold=self.feedback_threshold)
+        eng = self.engine
+        idx_d = eng.upload(np.ascontiguousarray(_as_index_array(idx)))
+        return eng.coo_to_csr(idx_d[:, 0], idx_d[:, 1], eng.upload(_as_value_array(val)), shape, drop_zeros=True)
+
+    def build(self, *args, **kwargs):
+        self._check_device_pmf(args, kwargs)
+        eng = self.engine
+        t0 = time.perf_counter()
+        a = self._pmf_training_csr()
+        n_users, n_items = a.shape
+        rank = int(self.rank)
+        plan = eng.sgd_plan(a, max(1, min(int(self.sgd_strata), n_users, n_items)))
+        del a
+        # initial factors: the reference's calls on the host (lib/optimize.py:173-175)
+        rnds = np.random if self.seed is None else np.random.RandomState(self.seed)
+        p_host = rnds.normal(scale=0.1, size=(n_users, rank))
+        q_host = rnds.normal(scale=0.1, size=(n_items, rank))
+        ld = round_up(rank, 32)
+        p = eng.zeros((n_users, ld), torch.float64)
+        q = eng.zeros((n_items, ld), torch.float64)
+        p[:, :rank].copy_(torch.from_numpy(p_host))
+        q[:, :rank].copy_(torch.from_numpy(q_host))
+        lam = 0.5 * self.sigma ** 2
+        self.rmse_history = []
+        self.iterations_time = []
+        last_err = np.finfo("f8").max
+        t1 = time.perf_counter()
+        for epoch in range(self.num_epochs):
+            te = time.perf_counter()
+            new_err = eng.sgd_epoch(plan, p, q, rank, self.learn_rate, lam)       # synchronises
+            self.iterations_time.append(time.perf_counter() - te)
+            refined = abs(last_err - new_err) / last_err
+            last_err = new_err
+            rmse = np.sqrt(new_err / plan.nnz)
+            self.rmse_history.append(rmse)
+            if self.show_rmse:
+                print("Epoch: {}. RMSE: {}".format(epoch, rmse))
+            if refined < self.tolerance:
+                break
+        t2 = time.perf_counter()
+        if self.training_time is not None:
+            self.training_time.append(t2 - t0)
+        if self.verbose:
+            print("{} training time: {:.3f}s".format(self.method, t2 - t0))
+        f = self.data.fields
+        self.factors[f.userid] = p[:, :rank].cpu().numpy()
+        self.factors[f.itemid] = q[:, :rank].cpu().numpy()
+        self.last_timings = dict(prepare_s=t1 - t0, sgd_s=t2 - t1, epochs=len(self.rmse_history), sgd_strata=plan.strata)
+        self._sgd_plan = plan              # kept for inspection (the permutation a build applied)
+
+    def _user_rows_device(self, test_users):
+        """fp32 copy of ``P[test_users]`` padded to 32 columns (the fused kernel's operand layout)."""
+        return self.engine.upload(_padded_f32(self.factors[self.data.fields.userid][np.asarray(test_users)]))
+
+    def get_recommendations(self):
+        if self.data.warm_start:
+            raise NotImplementedError                               # models.py:772-776
+        if self.verify_integrity and hasattr(self, "verify_data_integrity"):
+            self.verify_data_integrity()
+        eng = self.engine
+        f = self.data.fields
+        test_data, shape, test_users = self._get_test_data()
+        if self.topk > shape[1]:
+            raise ValueError("topk exceeds the number of items")
+        _, seen = self._test_csr_device(test_data, shape)
+        e = self._user_rows_device(test_users)
+        v_dev = self._device_factor(f.itemid)
+        if self.score_kernel is not None:
+            eng.set_score_kernel(self.score_kernel)
+        ids = eng.score_topk(e, v_dev, self.factors[f.itemid].shape[1], self.topk,
+                             seen=seen if self.filter_seen else None)
+        return ids.cpu().numpy()
+
+    def slice_recommendations(self, test_data, shape, start, stop, test_users=None):
+        """Dense score rows ``P[test_users[start:stop]] Q^T`` for a (small) user slice (models.py:779-787).  Returns
+        ``(scores float64 [m x n_items], slice_data)``; without ``test_users`` (what ``_user_scores`` passes) they are
+        taken from the test data."""
+        if test_users is None:
+            test_users = self._get_test_data()[2]
+        user, item, fdbk = (np.asarray(x) for x in test_data)
+        sel = (user >= start) & (user < stop)
+        sl = (user[sel] - start, item[sel], fdbk[sel])
+        f = self.data.fields
+        e = self._user_rows_device(np.asarray(test_users)[start:stop])
+        v_dev = self._device_factor(f.itemid)
+        s = self.engine.score_dense(e, v_dev, self.factors[f.itemid].shape[1])
+        return s.cpu().numpy().astype(np.float64), sl
+
+
+class B200ProbabilisticMF(_PMFDeviceMixin, host.RecommenderModel):
+    """ProbabilisticMF (models.py:728-787) on the device, standalone.  ``optimizer = None`` stands for the reference's
+    ``simple_pmf_sgd``, the only one on the device path."""
+
+    def __init__(self, *args, **kwargs):
+        self.seed = kwargs.pop("seed", None)
+        super().__init__(*args, **kwargs)
+        self.method = "PMF"
+        self.optimizer = None
+        self.learn_rate = 0.005
+        self.sigma = 1
+        self.num_epochs = 25
+        self.rank = 10
+        self.tolerance = 1e-4
+        self.factors = {}
+        self.rmse_history = None
+        self.show_rmse = False
+        self.iterations_time = None
+
+    def build(self, *args, **kwargs):
+        return _PMFDeviceMixin.build(self, *args, **kwargs)
+
+
+def dropin_pmf():
+    """``PolaraB200PMF``: the device path under the REAL ``polara`` ``ProbabilisticMF`` (requires the reference package
+    to be importable)."""
+    from polara.recommender.models import ProbabilisticMF
+
+    class PolaraB200PMF(_PMFDeviceMixin, ProbabilisticMF):
+        def build(self, *args, **kwargs):
+            return _PMFDeviceMixin.build(self, *args, **kwargs)
+
+    return PolaraB200PMF
 
 
 def dropin():
